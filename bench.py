@@ -8,6 +8,7 @@ Contract: `python bench.py --gpus N --steps K --warmup W` (N > 1 under torchrun)
             gradient inside the timed region)
   roofline  dominant kernel (largest share of the step), algorithmic bytes / CUDA-event time vs MEASURED_PEAKS.json
   cpu_baseline  the CPU oracle (restatement of torch-harmonics + makani einsums) on this box's host cores (bounded sample)
+`--dump-outputs DIR` writes the outputs of the last timed step (the inputs are seeded: two builds can be compared output for output).
 `--impl reference` times that CPU implementation alone (the reference has no other implementation of this path that can run
 here: torch-harmonics is not installable, see DESIGN.md).
 """
@@ -241,12 +242,12 @@ def run_reference_arm(args):
         return run_reference_model_arm(args)
     wl = args.workload
     cores, avail = pick_cpu_threads()
-    steps = max(1, min(args.steps, 3))  # bounded: each step is a full fwd+bwd of the workload (~10 s of CPU work)
-    t = cpu_reference_steps(wl, steps, min(args.warmup, 1))
+    steps = args.steps   # each step is a full fwd+bwd of the workload (~10 s of CPU work at the default workload)
+    t = cpu_reference_steps(wl, steps, args.warmup)
     val = 1.0 / t
     line = {
         "impl": "reference", "metric": "SFNO-block fwd+bwd samples/sec", "value": val, "unit": "samples/s", "n_gpus": args.gpus, "steps": steps,
-        "warmup": min(args.warmup, 1), "ms_per_step": t * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32",
+        "warmup": args.warmup, "ms_per_step": t * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32",
         "data": "synthetic", "config": {"workload": wl, "batch_per_gpu": 1, "activations": "bf16", "parallelism": "cpu"},
         "cpu_baseline": {"value": val, "unit": "samples/s", "cores": cores, "kind": "port",
                          "sample": f"{steps} full fwd+bwd steps of the workload through oracle/makani_oracle.py (torch.fft + torch.einsum, fp32, {cores} threads chosen by calibration of {avail} available)"},
@@ -257,7 +258,7 @@ def run_reference_arm(args):
 
 def run_reference_model_arm(args):
     """CPU arm of the full-model workloads: the same network (makani_b200.sfno, pinned against the reference's network class by
-    tests/golden/sfno_golden.npz) on the oracle transforms / SpectralConv, bf16 autocast off (CPU), one bounded step."""
+    tests/golden/sfno_golden_<case>.npz) on the oracle transforms / SpectralConv, bf16 autocast off (CPU), --warmup + --steps steps."""
     from makani_b200.sfno import SphericalFourierNeuralOperatorNet
     from oracle.sfno_backend import OracleBackend
 
@@ -266,18 +267,46 @@ def run_reference_model_arm(args):
     torch.manual_seed(333)
     net = SphericalFourierNeuralOperatorNet(**cfg, backend=OracleBackend())
     x = torch.randn(1, cfg["inp_chans"], *cfg["inp_shape"])
-    t0 = time.perf_counter()
-    out = net(x)
-    out.float().square().mean().backward()
-    t = time.perf_counter() - t0
+    times = []
+    for it in range(args.warmup + args.steps):
+        net.zero_grad(set_to_none=True)
+        t0 = time.perf_counter()
+        out = net(x)
+        out.float().square().mean().backward()
+        if it >= args.warmup:
+            times.append(time.perf_counter() - t0)
+    t = sum(times) / len(times)
     val = 1.0 / t
     print(json.dumps({
-        "impl": "reference", "metric": "SFNO model fwd+bwd samples/sec", "value": val, "unit": "samples/s", "n_gpus": args.gpus, "steps": 1, "warmup": 0,
+        "impl": "reference", "metric": "SFNO model fwd+bwd samples/sec", "value": val, "unit": "samples/s", "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
         "ms_per_step": t * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
         "config": {"workload": args.workload, "batch_per_gpu": 1, "parallelism": "cpu"},
         "cpu_baseline": {"value": val, "unit": "samples/s", "cores": cores, "kind": "port",
-                         "sample": f"1 full fwd+bwd step of the network on oracle/ (torch.fft + torch.einsum, fp32, {cores} threads of {avail})"},
+                         "sample": f"{args.steps} full fwd+bwd steps of the network on oracle/ (torch.fft + torch.einsum, fp32, {cores} threads of {avail})"},
         "e2e": {"value": val, "unit": "samples/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}), flush=True)
+
+
+DUMP_SAMPLE = 1 << 22    # --dump-outputs: elements kept of a larger output (a fixed, seeded sample)
+DUMP_GRAD_SAMPLE = 4096  # --dump-outputs, model workloads: elements kept of each parameter gradient
+
+
+def sample_flat(t, k, seed=0):
+    """t flattened to float32 on the host; when it has more than k elements, the same k of them on every run (seeded, sorted indices)"""
+    t = torch.view_as_real(t) if t.is_complex() else t
+    flat = t.detach().reshape(-1)
+    if flat.numel() <= k:
+        return t.detach().float().cpu()
+    idx = torch.randint(0, flat.numel(), (k,), generator=torch.Generator().manual_seed(seed)).sort().values
+    return flat[idx.to(flat.device)].float().cpu()
+
+
+def dump_outputs(out_dir, arrays):
+    """arrays: name -> tensor, each written as out_dir/<name>.npy (float32)"""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.numpy().astype(np.float32, copy=False))
 
 
 HXW_GRID = {2: (1, 2), 4: (2, 2), 8: (4, 2)}   # h x w spatial model-parallel grids (cfg 4 of BASELINE.json is h = 4, w = 2)
@@ -390,7 +419,7 @@ def run_gpu_arm(args):
     gw_host = torch.empty(conv.weight.shape, dtype=torch.complex64).pin_memory()
     flush = torch.empty(256 * 1024 * 1024, dtype=torch.uint8, device=dev)  # > 126 MB L2
 
-    def step(xin):
+    def step(xin, keep=None):
         xin.requires_grad_(True)
         conv.weight.grad = None
         y, _ = conv(xin)
@@ -398,6 +427,8 @@ def run_gpu_arm(args):
         g = xin.grad
         xin.grad = None
         xin.requires_grad_(False)
+        if keep is not None:   # --dump-outputs: what a caller of the step receives
+            keep.update(y=y.detach(), dx=g)
         return g
 
     def step_e2e():
@@ -504,8 +535,10 @@ def run_gpu_arm(args):
     if world > 1 and dp_mode == "overlap":
         conv.wgrad_ready_event = torch.cuda.Event()
 
+    last = {} if args.dump_outputs else None   # outputs of the latest timed step
+
     def dp_step():
-        step(x_dev)
+        step(x_dev, last)
         if world > 1 and dp_mode != "overlap":   # the all-reduce trails the backward pass on the compute stream (default communicator)
             dist.all_reduce(torch.view_as_real(conv.weight.grad))
         elif world > 1:
@@ -514,6 +547,8 @@ def run_gpu_arm(args):
                 dist.all_reduce(torch.view_as_real(conv.weight.grad), group=dp_group)
             conv.weight.grad.record_stream(side)
             torch.cuda.current_stream(dev).wait_stream(side)
+        if last is not None:
+            last["dweight"] = conv.weight.grad
 
     # kernel launches of OUR library inside one step (counted by the ctypes call wrapper)
     counter = {"n": 0}
@@ -555,6 +590,8 @@ def run_gpu_arm(args):
                 torch.cuda.synchronize()
         ms_dev = timed(dp_step, args.steps, args.warmup)
         host_ms = host_enqueue.get("ms_per_step")
+        dumped = {k: sample_flat(v, DUMP_SAMPLE) for k, v in last.items()} if (last is not None and rank == 0) else None
+        last = None
         # the same step replayed from a CUDA graph, reported separately (`value` stays the eager step: it is what N > 1 and e2e run)
         if args.graph and world == 1:
             graph_info = try_cuda_graph()
@@ -712,6 +749,8 @@ def run_gpu_arm(args):
         line["cuda_graph_replay"] = graph_info
     if hxw is not None:
         line["hxw"] = hxw
+    if dumped is not None:
+        dump_outputs(args.dump_outputs, dumped)
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -757,14 +796,18 @@ def run_model_arm(args):
     loss_host = torch.zeros(1).pin_memory()
     flush = torch.empty(256 * 1024 * 1024, dtype=torch.uint8, device=dev)
 
-    def step(xd):
+    def step(xd, keep=None):
         for p_ in net.parameters():
             p_.grad = None
         with torch.autocast(device_type="cuda", dtype=act_dtype, enabled=(act_dtype == torch.bfloat16)):
             out = net(xd)
         loss = out.float().square().mean()
         loss.backward()
+        if keep is not None:   # --dump-outputs: what a caller of the step receives (the parameter gradients are read after the timed loop)
+            keep.update(out=out.detach(), loss=loss.detach().reshape(1))
         return loss
+
+    last = {} if args.dump_outputs else None   # outputs of the latest timed step
 
     def timed(fn, steps, warmup):
         for _ in range(warmup):
@@ -818,7 +861,12 @@ def run_model_arm(args):
             while not sampler.lines and time.perf_counter() - t_wait < 5.0:
                 step(x_dev)
                 torch.cuda.synchronize()
-        ms = timed(lambda: step(x_dev), args.steps, args.warmup)
+        ms = timed(lambda: step(x_dev, last), args.steps, args.warmup)
+        dumped = None
+        if last is not None and rank == 0:
+            grads = [sample_flat(p_.grad, DUMP_GRAD_SAMPLE, seed=i).reshape(-1) for i, (_, p_) in enumerate(net.named_parameters()) if p_.grad is not None]
+            dumped = {"out": sample_flat(last["out"], DUMP_SAMPLE), "loss": last["loss"].float().cpu(), "param_grads": torch.cat(grads)}
+        last = None
         clocks = sampler.stop() if sampler else None
         ms_e2e = timed(step_e2e, args.steps, max(1, args.warmup // 2))
     finally:
@@ -868,6 +916,8 @@ def run_model_arm(args):
         "cpu_baseline": None,
         "gpu_library_baseline": lib,
     }
+    if dumped is not None:
+        dump_outputs(args.dump_outputs, dumped)
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -876,8 +926,10 @@ def run_model_arm(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
-    ap.add_argument("--warmup", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps of the measured step (`value`, also with --impl reference); the side measurements (roofline_stages, hxw, "
+                         "cpu_baseline, gpu_library_baseline) use their own small bounded counts")
+    ap.add_argument("--warmup", type=int, default=5, help="untimed steps before the timed ones")
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="sfno_block_721x1440x73", choices=sorted(WORKLOADS) + sorted(MODEL_WORKLOADS))
     ap.add_argument("--precision", default="best", choices=["best", "fp32", "tf32", "fp32x3"])
@@ -890,7 +942,14 @@ def main():
     ap.add_argument("--dp-mode", default=os.environ.get("B200SHT_DP_MODE", "trailing"), choices=["overlap", "trailing"],
                     help="N > 1: weight-gradient all-reduce after the backward pass on the compute stream (trailing, default: measured faster, DESIGN.md section 7) or on a "
                          "side stream behind the wgrad event with reserved SMs (overlap)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (float32): block workloads y, dx, dweight; model workloads "
+                         f"out, loss, param_grads; outputs over {DUMP_SAMPLE} elements as a fixed seeded sample of that many")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the CUDA path (--impl b200)")
     if args.impl == "reference":
         run_reference_arm(args)
     else:

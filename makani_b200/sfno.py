@@ -4,7 +4,7 @@ Restates, with the same constructor arguments, parameter names, shapes, initiali
   NeuralOperatorBlock                 makani/models/networks/sfnonet.py:169-408   (filter -> norm0 -> [+inner skip] -> act -> MLP -> norm1 -> drop path -> [+outer skip])
   SphericalFourierNeuralOperatorNet   makani/models/networks/sfnonet.py:411-934   (encoder, position embedding, blocks, decoder, big skip; `_init_spectral_transforms` :765-838)
   MLP / EncoderDecoder                makani/models/common/layers.py:537-760      (1x1-convolution stacks, `fwd` Sequential)
-so that a checkpoint of the reference network loads with `load_state_dict(strict=True)` and gives the same outputs (tests/golden/sfno_golden.npz is
+so that a checkpoint of the reference network loads with `load_state_dict(strict=True)` and gives the same outputs (tests/golden/sfno_golden_<case>.npz is
 produced by the REFERENCE class here, tests/golden/make_sfno_golden.py).  Single-process (h = w = 1) SHT variant; the makani package itself can also
 be run unchanged on these kernels through makani_b200.compat (torch_harmonics shim).
 

@@ -5,7 +5,7 @@ with the reference's own SpectralConv / MLP / EncoderDecoder, run on the CPU ora
 (tests/reference_suites/run_reference_tests.py::install_environment).  Stored per case: the full state dict, the input, the output,
 d(loss)/d(input) and the gradients of a few parameters for loss = sum(out * g).
 
-    python tests/golden/make_sfno_golden.py        # needs /root/reference (build container only) -> tests/golden/sfno_golden.npz
+    MAKANI_REFERENCE=<makani checkout> python tests/golden/make_sfno_golden.py   -> tests/golden/sfno_golden_<case>.npz (one file per case)
 """
 import os
 import sys
@@ -61,9 +61,10 @@ def main():
             gr = params[k].grad
             out[f"{name}/grad/{k}"] = torch.view_as_real(gr).numpy() if gr.is_complex() else gr.numpy()
         print(name, "params", sum(p.numel() for p in net.parameters()), "y", tuple(y.shape), "|y|", float(y.abs().mean()))
-    path = os.path.join(HERE, "sfno_golden.npz")
-    np.savez_compressed(path, **out)
-    print("wrote", path, os.path.getsize(path), "bytes")
+    for name in SFNO_GOLDEN_CASES:
+        path = os.path.join(HERE, f"sfno_golden_{name}.npz")
+        np.savez_compressed(path, **{k: v for k, v in out.items() if k.startswith(name + "/")})
+        print("wrote", path, os.path.getsize(path), "bytes")
 
 
 if __name__ == "__main__":

@@ -13,7 +13,11 @@ execute from where they lie.  These are the known-answer tests the reference hol
     python tests/reference_suites/run_reference_tests.py            # prints one line per class, exit code 1 on any failure
     python tests/reference_suites/run_reference_tests.py --report   # also rewrites tests/reference_suites/report.txt
 
-Only runs where /root/reference is mounted (the build container); tests/test_reference_suites.py wraps it for pytest.
+    python tests/reference_suites/run_reference_tests.py --record tests/golden/reference_sht_boundary.npz
+                                                                    # also stores the calls the suites make into the stand-ins
+
+The reference tree is taken from $MAKANI_REFERENCE (a checkout of makani).  The recorded calls are replayed without it by
+tests/test_reference_suites.py.
 """
 import importlib
 import inspect
@@ -25,7 +29,7 @@ import unittest
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-REF = "/root/reference"
+REF = os.environ.get("MAKANI_REFERENCE", "")
 
 # reference test classes that go through torch_harmonics.{RealSHT, InverseRealSHT, quadrature}
 SUITES = {
@@ -145,9 +149,85 @@ def install_environment():
     sys.modules.setdefault("parameterized", par)
 
 
-def run():
-    """-> list of (module, class, ran, failures, errors, [messages])"""
+MAX_CALLS_PER_KEY = 2          # recorded calls per distinct transform / quadrature call
+MAX_SLICE_ELEMS = 1 << 14      # larger transform slices are not recorded (file size)
+QUADRATURE_FNS = ("legendre_gauss_weights", "clenshaw_curtiss_weights", "precompute_latitudes", "precompute_longitudes")
+
+
+def install_recorder(transforms, quadrature):
+    """Wrap the stand-ins installed as torch_harmonics: per distinct transform (constructor arguments, table and input dtype) the first
+    MAX_CALLS_PER_KEY inputs and outputs are kept, reduced to the leading [0, ..., 0] slice (the transforms act on the last two
+    dimensions only); per distinct quadrature call its outputs."""
+    import json
+
+    from oracle import makani_oracle as O
+
+    th = sys.modules["torch_harmonics"]
+
+    def wrap(base, kind, table):
+        class Recording(base):
+            def forward(self, x):
+                y = super().forward(x)
+                key = json.dumps([kind, self.nlat, self.nlon, self.lmax, self.mmax, self.grid, self.csphase,
+                                  str(getattr(self, table).dtype), str(x.dtype)])
+                xs, ys = x.detach().reshape(-1, *x.shape[-2:])[0], y.detach().reshape(-1, *y.shape[-2:])[0]
+                calls = transforms.setdefault(key, [])
+                if len(calls) < MAX_CALLS_PER_KEY and xs.numel() <= MAX_SLICE_ELEMS and ys.numel() <= MAX_SLICE_ELEMS:
+                    calls.append((xs.clone(), ys.clone()))
+                return y
+
+        Recording.__name__ = base.__name__
+        return Recording
+
+    th.RealSHT = wrap(O.RealSHT, "RealSHT", "weights")
+    th.InverseRealSHT = wrap(O.InverseRealSHT, "InverseRealSHT", "pct")
+    quad = types.ModuleType("torch_harmonics.quadrature")
+    quad.__dict__.update({k: v for k, v in vars(th.quadrature).items() if not k.startswith("__")})
+
+    def wrap_fn(name, fn):
+        def g(*a, **k):
+            r = fn(*a, **k)
+            key = json.dumps([name, list(a), sorted(k.items())])
+            if key not in quadrature:
+                quadrature[key] = [t.clone() for t in (r if isinstance(r, tuple) else (r,))]
+            return r
+        return g
+
+    for name in QUADRATURE_FNS:
+        if hasattr(quad, name):
+            setattr(quad, name, wrap_fn(name, getattr(quad, name)))
+    th.quadrature = quad
+    sys.modules["torch_harmonics.quadrature"] = quad
+
+
+def save_recording(path, transforms, quadrature):
+    """npz: `meta` (JSON: one [key, n_calls] per transform, one [key, n_outputs] per quadrature call) and the arrays
+    t{i}/{j}/x, t{i}/{j}/y, q{i}/{j}; complex arrays are stored as (..., 2) real views."""
+    import json
+
+    import numpy as np
+
+    def arr(t):
+        return (torch.view_as_real(t) if t.is_complex() else t).numpy()
+
+    data, meta = {}, {"transforms": [], "quadrature": []}
+    for i, (key, calls) in enumerate(sorted(transforms.items())):
+        meta["transforms"].append([key, len(calls)])
+        for j, (x, y) in enumerate(calls):
+            data[f"t{i}/{j}/x"], data[f"t{i}/{j}/y"] = arr(x), arr(y)
+    for i, (key, outs) in enumerate(sorted(quadrature.items())):
+        meta["quadrature"].append([key, len(outs)])
+        for j, t in enumerate(outs):
+            data[f"q{i}/{j}"] = arr(t)
+    data["meta"] = np.array(json.dumps(meta))
+    np.savez_compressed(path, **data)
+
+
+def run(record=None):
+    """-> list of (module, class, ran, failures, errors, [messages]); record: (transforms, quadrature) dicts filled by install_recorder"""
     install_environment()
+    if record is not None:
+        install_recorder(*record)
     results = []
     for modname, classes in SUITES.items():
         M = importlib.import_module(modname)
@@ -161,9 +241,12 @@ def run():
 
 def main():
     if not os.path.isdir(REF):
-        print("reference tree not mounted: nothing to run")
+        print("reference tree not found (set MAKANI_REFERENCE): nothing to run")
         return 0
-    results = run()
+    record = ({}, {}) if "--record" in sys.argv else None
+    results = run(record)
+    if record is not None:
+        save_recording(sys.argv[sys.argv.index("--record") + 1], *record)
     lines = []
     for modname, name, ran, nf, ne, msgs in results:
         lines.append(f"{modname}.{name}: ran {ran}  failures {nf}  errors {ne}")
@@ -174,7 +257,7 @@ def main():
     print("\n".join(lines))
     if "--report" in sys.argv:
         with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "report.txt"), "w") as f:
-            f.write("python tests/reference_suites/run_reference_tests.py --report   (reference tree at /root/reference)\n" + "\n".join(lines) + "\n")
+            f.write("python tests/reference_suites/run_reference_tests.py --report   (reference tree at $MAKANI_REFERENCE)\n" + "\n".join(lines) + "\n")
     return 1 if bad else 0
 
 

@@ -1,6 +1,6 @@
 """SURVEY rows A8 / A9 on the GPU: the SFNO network (makani_b200/sfno.py: NeuralOperatorBlock, SphericalFourierNeuralOperatorNet) running on the
 CUDA spherical-harmonic kernels, loaded with the REFERENCE network's state dict and compared with the REFERENCE network's output and gradients
-(tests/golden/sfno_golden.npz, produced by /root/reference/makani/models/networks/sfnonet.py on the CPU oracle, tests/golden/make_sfno_golden.py)."""
+(tests/golden/sfno_golden_<case>.npz, produced by makani's makani/models/networks/sfnonet.py on the CPU oracle, tests/golden/make_sfno_golden.py)."""
 import os
 import sys
 
@@ -13,7 +13,7 @@ from test_gpu_parity import close
 
 sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
 from make_sfno_golden import GRAD_KEYS, SFNO_GOLDEN_CASES  # noqa: E402
-from test_sfno_cpu import GOLD, golden_state_dict  # noqa: E402
+from test_sfno_cpu import golden_state_dict, load_golden  # noqa: E402
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda"
@@ -35,7 +35,7 @@ def test_sfno_network_matches_reference_network(name, precision, rtol, grtol, to
     transform pair and block (+ cuDNN TF32 convolutions), amplified through the instance norms in the gradients (grtol).  The ReLU network
     ("plain") is compared in its output only at TF32: a 1e-3 perturbation flips ReLU gates, its gradient is not a continuous function."""
     torch.backends.cuda.matmul.allow_tf32 = torch.backends.cudnn.allow_tf32 = (precision == "tf32")
-    g = np.load(GOLD)
+    g = load_golden(name)
     net = SphericalFourierNeuralOperatorNet(**SFNO_GOLDEN_CASES[name], precision=precision)
     net.load_state_dict(golden_state_dict(g, name), strict=True)
     net = net.to(DEV)
@@ -58,7 +58,7 @@ def test_sfno_network_matches_reference_network(name, precision, rtol, grtol, to
 def test_sfno_network_bf16_autocast_runs_and_is_close():
     """the way the reference trains (bf16 autocast around the network; the transforms stay fp32/TF32): loose agreement with the fp32 golden output"""
     name = "sc3_base"
-    g = np.load(GOLD)
+    g = load_golden(name)
     net = SphericalFourierNeuralOperatorNet(**SFNO_GOLDEN_CASES[name], precision="tf32")
     net.load_state_dict(golden_state_dict(g, name), strict=True)
     net = net.to(DEV)

@@ -14,7 +14,12 @@ from oracle.sfno_backend import OracleBackend
 sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
 from make_sfno_golden import GRAD_KEYS, SFNO_GOLDEN_CASES  # noqa: E402
 
-GOLD = os.path.join(os.path.dirname(__file__), "golden", "sfno_golden.npz")
+GOLDEN_DIR = os.path.join(os.path.dirname(__file__), "golden")
+
+
+def load_golden(name):
+    """the arrays of one case (keys `<name>/...`), one file per case to keep each file small"""
+    return np.load(os.path.join(GOLDEN_DIR, f"sfno_golden_{name}.npz"))
 
 
 def golden_state_dict(g, name):
@@ -29,7 +34,7 @@ def golden_state_dict(g, name):
 
 @pytest.mark.parametrize("name", sorted(SFNO_GOLDEN_CASES))
 def test_network_on_oracle_backend_matches_reference_network(name):
-    g = np.load(GOLD)
+    g = load_golden(name)
     torch.manual_seed(0)
     net = SphericalFourierNeuralOperatorNet(**SFNO_GOLDEN_CASES[name], backend=OracleBackend())
     sd = golden_state_dict(g, name)
@@ -51,7 +56,7 @@ def test_network_on_oracle_backend_matches_reference_network(name):
 @pytest.mark.parametrize("name", sorted(SFNO_GOLDEN_CASES))
 def test_cuda_backed_network_has_the_reference_parameter_surface(name):
     """constructed on CPU (plans are created lazily on the device): names, shapes, dtypes of every state-dict entry, and the checkpoint loads"""
-    g = np.load(GOLD)
+    g = load_golden(name)
     net = SphericalFourierNeuralOperatorNet(**SFNO_GOLDEN_CASES[name], precision="fp32")
     sd = golden_state_dict(g, name)
     mine = net.state_dict()
