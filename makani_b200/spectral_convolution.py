@@ -207,6 +207,10 @@ class _SpectralConvOneCall(torch.autograd.Function):
         if need_w:
             gw = torch.empty(wshape, dtype=torch.complex64, device=dev) if op in _DENSE_OPS else gw_dev
         ev = ctx.wgrad_event
+        if ev is not None and not ev.cuda_event:
+            # torch creates the CUDA event at its first record: without a handle the library would see no event, skip the overlapped
+            # schedule, and a stream waiting on the event would not wait for the gradient at all
+            ev.record(torch.cuda.current_stream(dev))
         _lib.call("b200sht_spectral_conv_backward_ex", pf.handle, pi.handle, dptr, _ptr(gy), _ptr(gres), _ptr(spec_saved), _ptr(wdev), _ptr(gx), _ptr(gw_dev),
                   _ptr(gb), _ptr(ws), _ptr(gw) if (need_w and op in _DENSE_OPS) else _VP(0), _VP(ev.cuda_event) if ev is not None else _VP(0), _stream(dev))
         gbias = gb.reshape(binfo[0]).to(binfo[1]) if need_b else None

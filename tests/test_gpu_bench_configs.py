@@ -42,23 +42,31 @@ def test_benched_block_strict_fp32():
         assert v < 5e-6, (k, rel)
 
 
-@pytest.mark.parametrize("chunks", [2, 3])
-def test_benched_block_latitude_chunked_analysis(chunks):
+@pytest.mark.parametrize("chunks,act_dtype", [pytest.param(2, torch.float32, id="2"), pytest.param(3, torch.float32, id="3"),
+                                              pytest.param(2, torch.bfloat16, id="2-bf16"), pytest.param(3, torch.bfloat16, id="3-bf16")])
+def test_benched_block_latitude_chunked_analysis(chunks, act_dtype):
     """The latitude-chunked (longitude analysis -> Legendre analysis) pair (b200sht_debug_set_lat_chunks; DESIGN.md section 10): same
-    tolerances against the oracle as the unchunked path, and agreement with it up to the summation order of the Legendre sums."""
+    tolerances against the oracle as the unchunked path, and agreement with it up to the summation order of the Legendre sums.  bf16
+    activations run the DFT's bf16 loader from a latitude offset."""
     from makani_b200 import _lib
 
     lib = _lib.load()
     old = lib.b200sht_debug_set_lat_chunks(1)
     try:
-        ref = _run_conv_case(CFG_2C, "tf32", 1e-3, act_dtype=torch.float32, return_outputs=True)
+        ref = _run_conv_case(CFG_2C, "tf32", 1e-3, act_dtype=act_dtype, return_outputs=True)
         lib.b200sht_debug_set_lat_chunks(chunks)
-        got = _run_conv_case(CFG_2C, "tf32", 1e-3, act_dtype=torch.float32, return_outputs=True)
+        got = _run_conv_case(CFG_2C, "tf32", 1e-3, act_dtype=act_dtype, return_outputs=True)
     finally:
         lib.b200sht_debug_set_lat_chunks(old)
+    bf16 = act_dtype == torch.bfloat16
     for k in ref[1]:
         a, b = got[1][k].double(), ref[1][k].double()
         d = float((a - b).norm() / b.norm())
-        print(f"[chunked x{chunks}] {k}: rel_l2 vs unchunked {d:.2e}, vs oracle {got[0][k]:.2e} (unchunked {ref[0][k]:.2e})")
-        assert d < 5e-4, (k, d)      # measured 1.5e-4: different summation order + TF32 rounding flips of the coefficients, below the 7e-4 error against the oracle
-        assert got[0][k] < 1e-3, (k, got[0])
+        print(f"[chunked x{chunks} {act_dtype}] {k}: rel_l2 vs unchunked {d:.2e}, vs oracle {got[0][k]:.2e} (unchunked {ref[0][k]:.2e})")
+        if bf16 and k != "dweight":
+            # bf16 outputs: the fp32 differences above flip a few percent of the bf16 roundings (one bf16 unit is 2^-8 relative)
+            assert d < 2e-3, (k, d)
+            assert got[0][k] < 3e-3, (k, got[0])
+        else:
+            assert d < 5e-4, (k, d)      # measured 1.5e-4: different summation order + TF32 rounding flips of the coefficients, below the 7e-4 error against the oracle
+            assert got[0][k] < (1.5e-3 if bf16 else 1e-3), (k, got[0])

@@ -10,6 +10,7 @@ import torch
 import makani_b200 as mb
 from makani_b200 import _lib
 from oracle import makani_oracle as O
+from test_gpu_dispatch import kernels_run, ran
 from test_gpu_parity import close
 
 pytestmark = pytest.mark.gpu
@@ -28,10 +29,52 @@ CASES = [
     (7, 1512, 256, 2, torch.float32),      # largest supported length class (N2 = 189, odd)
     (19, 16, 9, 3, torch.float32),         # smallest
 ]
+# The analysis kernel reads fp32 rows only when nlon % 32 == 0 (16-byte TMA boxes; otherwise fft_analysis runs the Stockham FFT):
+# test_dft_analysis_gpu runs the other fp32 entries of CASES as bf16.  Its further cases cover the analysis variants of dft.cu --
+# bf16 box groups gs = 1 / 4 / 8 (dft_box_group), one / two / three K-blocks (N2/2 + 1 <= 32 / 64 / 96), the N2 = 90 specialisation --
+# at ragged nlat, with mmax truncated or up to the Nyquist order.
+ANALYSIS_CASES = [
+    (7, 16, 9, 3, torch.bfloat16),         # N2 = 2, gs 4, Nyquist
+    (45, 16, 5, 2, torch.bfloat16),
+    (19, 72, 37, 3, torch.bfloat16),       # N2 = 9 (odd), gs 8, 4 replicas, Nyquist
+    (181, 72, 20, 2, torch.bfloat16),
+    (45, 128, 65, 2, torch.bfloat16),      # gs 1, Nyquist
+    (7, 128, 30, 3, torch.bfloat16),
+    (181, 720, 241, 2, torch.bfloat16),    # N2 = 90 template, gs 4, two K-blocks: the 360 x 720 inner grid of SFNO scale_factor 2
+    (19, 720, 256, 3, torch.bfloat16),
+    (7, 1024, 256, 2, torch.bfloat16),     # gs 1, three K-blocks
+    (45, 1024, 100, 3, torch.bfloat16),
+    (19, 1512, 256, 2, torch.bfloat16),    # N2 = 189 (odd, largest), gs 8, three K-blocks
+    (181, 1512, 121, 2, torch.bfloat16),
+    (45, 256, 129, 3, torch.float32),      # Nyquist
+    (181, 256, 60, 2, torch.float32),
+    (19, 1024, 256, 2, torch.float32),     # three K-blocks
+    (7, 1024, 33, 3, torch.float32),
+]
 
 
 def _latview(lat, plan, B, C, mmax):
     return lat[: mmax * 2 * B * C * plan.kp].view(mmax, 2, B * C, plan.kp)
+
+
+def _analysis_vs_rfft(lat, x, plan, mode, rtol, name):
+    """latspec written by b200sht_fft_analysis (scale mode 0 or 1) against 2 pi rfft in fp64 (mode 0: times the quadrature weights)"""
+    B, C, nlat, nlon = x.shape
+    mmax = plan.mmax
+    X = _latview(lat, plan, B, C, mmax)
+    got = torch.complex(X[:, 0, :, :nlat], X[:, 1, :, :nlat]).permute(1, 2, 0).reshape(B, C, nlat, mmax)
+    assert (X[..., nlat:] == 0).all(), "latitude padding must hold exact zeros"
+    ref = torch.fft.rfft(x.double().cpu(), dim=-1)[..., :mmax]
+    if mode == 0:
+        _, w = O.precompute_latitudes(nlat, "equiangular")
+        ref = ref * (torch.from_numpy(w) * 2 * math.pi / nlon)[:, None]
+    else:
+        ms = torch.full((mmax,), 2.0, dtype=torch.float64)
+        ms[0] = 1
+        if mmax - 1 == nlon // 2:
+            ms[-1] = 1
+        ref = ref * ms
+    return close(got, ref, rtol, name)
 
 
 def to_tiled(Z, plan):
@@ -45,32 +88,66 @@ def to_tiled(Z, plan):
     return Zp.view(M2, 8, 2, R, kp // 8, 8).permute(3, 4, 2, 0, 1, 5).contiguous().reshape(-1)
 
 
-@pytest.mark.parametrize("nlat,nlon,mmax,C,dtype", CASES)
+@pytest.mark.parametrize("nlat,nlon,mmax,C,dtype", CASES + ANALYSIS_CASES)
 def test_dft_analysis_gpu(nlat, nlon, mmax, C, dtype):
+    if dtype == torch.float32 and nlon % 32:
+        dtype = torch.bfloat16
     torch.manual_seed(333)
     plan = mb.get_plan(nlat, nlon, min(nlat, 16), mmax, "equiangular", True, torch.device(DEV))
-    assert plan.query(8) == 1, "tensor-core DFT not available for this grid"
     B = 2
     x = torch.randn(B, C, nlat, nlon, device=DEV).to(dtype)
     st = mb.sht._stream(x.device)
+    N2 = nlon // 8
     for mode in (0, 1):
         lat = torch.full((plan.latspec_elems(B, C),), float("nan"), device=DEV)
-        _lib.call("b200sht_fft_analysis", plan.handle, mb.sht._ptr(x), mb.sht._dtype_code(dtype), B, C, mb.sht._ptr(lat), mode | 2, st)
-        X = _latview(lat, plan, B, C, mmax)
-        got = torch.complex(X[:, 0, :, :nlat], X[:, 1, :, :nlat]).permute(1, 2, 0).reshape(B, C, nlat, mmax)
-        assert (X[..., nlat:] == 0).all(), "latitude padding must hold exact zeros"
-        ref = torch.fft.rfft(x.double().cpu(), dim=-1)[..., :mmax]
-        if mode == 0:
-            _, w = O.precompute_latitudes(nlat, "equiangular")
-            ref = ref * (torch.from_numpy(w) * 2 * math.pi / nlon)[:, None]
-        else:
-            ms = torch.full((mmax,), 2.0, dtype=torch.float64)
-            ms[0] = 1
-            if mmax - 1 == nlon // 2:
-                ms[-1] = 1
-            ref = ref * ms
-        rel = close(got, ref, 1e-3, f"dft_analysis mode{mode} {nlat}x{nlon} mmax={mmax} {dtype}")
+        _, names = kernels_run(lambda: _lib.call("b200sht_fft_analysis", plan.handle, mb.sht._ptr(x), mb.sht._dtype_code(dtype), B, C, mb.sht._ptr(lat),
+                                                 mode | 2, st))
+        assert ran(names, "dft_analysis_kernel<", f", {N2 if N2 in (60, 90, 180) else 0}>"), names
+        rel = _analysis_vs_rfft(lat, x, plan, mode, 1e-3, f"dft_analysis mode{mode} {nlat}x{nlon} mmax={mmax} {dtype}")
         assert rel < 6e-4, rel
+
+
+def test_fp32_input_at_nlon_720_runs_stockham_rounded_to_tf32():
+    """fp32 rows of 720 samples cannot be read by the DFT's TMA boxes: with the TF32 bit the Stockham FFT runs and rounds its output to
+    TF32 (it feeds the tcgen05 Legendre GEMM)"""
+    torch.manual_seed(335)
+    nlat, nlon, mmax, B, C = 45, 720, 241, 2, 3
+    plan = mb.get_plan(nlat, nlon, 16, mmax, "equiangular", True, torch.device(DEV))
+    assert plan.query(8) == 1
+    x = torch.randn(B, C, nlat, nlon, device=DEV)
+    st = mb.sht._stream(x.device)
+    for mode in (0, 1):
+        lat = torch.full((plan.latspec_elems(B, C),), float("nan"), device=DEV)
+        _, names = kernels_run(lambda: _lib.call("b200sht_fft_analysis", plan.handle, mb.sht._ptr(x), 0, B, C, mb.sht._ptr(lat), mode | 2, st))
+        assert ran(names, "fft_analysis_") and not ran(names, "dft_analysis_kernel"), names
+        X = _latview(lat, plan, B, C, mmax)
+        assert (X.view(torch.int32) & 0x1FFF == 0).all(), "output not rounded to TF32"
+        rel = _analysis_vs_rfft(lat, x, plan, mode, 1e-3, f"stockham+tf32 mode{mode} {nlat}x{nlon} fp32")
+        assert rel < 6e-4, rel
+
+
+def test_misaligned_bf16_input_runs_stockham():
+    """bf16 721 x 1440 samples 2 bytes off a 16-byte boundary: TMA cannot address them, the Stockham FFT runs -- through the C ABI and
+    through RealSHT(precision="tf32") on a contiguous view with a storage offset"""
+    torch.manual_seed(336)
+    nlat, nlon, lmax, mmax, B, C = 721, 1440, 240, 241, 1, 2
+    plan = mb.get_plan(nlat, nlon, lmax, mmax, "equiangular", True, torch.device(DEV))
+    assert plan.query(8) == 1
+    buf = torch.randn(B * C * nlat * nlon + 1, device=DEV).to(torch.bfloat16)
+    x = buf[1:].view(B, C, nlat, nlon)
+    assert x.is_contiguous() and x.data_ptr() % 16 == 2
+    st = mb.sht._stream(x.device)
+    lat = torch.full((plan.latspec_elems(B, C),), float("nan"), device=DEV)
+    _, names = kernels_run(lambda: _lib.call("b200sht_fft_analysis", plan.handle, mb.sht._ptr(x), _lib.BF16, B, C, mb.sht._ptr(lat), 0 | 2, st))
+    assert ran(names, "fft_analysis_") and not ran(names, "dft_analysis_kernel"), names
+    rel = _analysis_vs_rfft(lat, x, plan, 0, 1e-3, f"misaligned bf16 fft_analysis {nlat}x{nlon}")
+    assert rel < 6e-4, rel
+    sht = mb.RealSHT(nlat, nlon, lmax, mmax, "equiangular", precision="tf32")
+    c, names = kernels_run(lambda: sht(x))
+    assert ran(names, "fft_analysis_") and not ran(names, "dft_analysis_kernel"), names
+    assert ran(names, "umma_kernel", "AnaTraits"), names
+    rel = close(c, O.RealSHT(nlat, nlon, lmax, mmax, "equiangular", dtype=torch.float64)(x.double().cpu()), 1e-3, "misaligned bf16 RealSHT tf32")
+    assert rel < 1e-3, rel
 
 
 @pytest.mark.parametrize("nlat,nlon,mmax,C,dtype", CASES)
@@ -88,7 +165,9 @@ def test_dft_synthesis_gpu(nlat, nlon, mmax, C, dtype):
     bias = torch.randn(C, device=DEV)
     Zc = torch.complex(Z[:, 0, :, :nlat], Z[:, 1, :, :nlat]).permute(1, 2, 0).reshape(B, C, nlat, mmax).to(torch.complex128).cpu()
     y = torch.full((B, C, nlat, nlon), float("nan"), device=DEV, dtype=dtype)
-    _lib.call("b200sht_fft_synthesis", plan.handle, mb.sht._ptr(lat), mb.sht._ptr(y), mb.sht._dtype_code(dtype), B, C, mb.sht._ptr(bias), 0 | 2, st)
+    _, names = kernels_run(lambda: _lib.call("b200sht_fft_synthesis", plan.handle, mb.sht._ptr(lat), mb.sht._ptr(y), mb.sht._dtype_code(dtype), B, C,
+                                             mb.sht._ptr(bias), 0 | 2, st))
+    assert ran(names, "dft_synthesis_kernel<"), names
     ref = torch.fft.irfft(Zc, n=nlon, dim=-1, norm="forward") + bias.double().cpu()[None, :, None, None]
     rel = close(y, ref, 1e-3 if dtype == torch.float32 else 4e-3, f"dft_synthesis mode0 {nlat}x{nlon} mmax={mmax} {dtype}")
     assert rel < (6e-4 if dtype == torch.float32 else 3e-3), rel
